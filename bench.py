@@ -69,7 +69,30 @@ def parse_args():
     ap.add_argument("--skip-cli", action="store_true")
     ap.add_argument("--cli-files", type=int, default=1000, help="FASTA files in the file -> .msh side measurement of the host shim")
     ap.add_argument("--cli-dist-sketches", type=int, default=6000, help="sketches in the `mash dist` wall-clock side measurement of the host shim")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed sketch step returned on rank 0 to DIR/*.npy (see dump_sketch_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_UNITS = 2048       # sketches whose hashes --dump-outputs writes: 2048 x 1000 hashes x 2 halves x 8 B = 33 MB
+
+
+def dump_sketch_outputs(out_dir, d_hashes, d_n):
+    """--dump-outputs: the result of the last timed sketch step, as float64 .npy files that hold every value exactly, so that two
+    builds can be compared output for output.  sketch_n_hashes = hashes in each unit's sketch (all units); for a fixed, seeded
+    sample of units (sketch_units, ascending), sketch_hashes_hi / _lo = the high and low 32 bits of their hashes (a uint64 does
+    not fit a float64).  Positions past a unit's count hold no result and are written as 0."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = d_n.cpu().numpy().astype(np.int64)
+    units = np.sort(np.random.Generator(np.random.PCG64(7)).choice(n.size, min(n.size, DUMP_UNITS), replace=False))
+    h = d_hashes.cpu().numpy().view(np.uint64)[units]
+    h[np.arange(h.shape[1])[None, :] >= n[units][:, None]] = 0
+    np.save(os.path.join(out_dir, "sketch_units.npy"), units.astype(np.float64))
+    np.save(os.path.join(out_dir, "sketch_n_hashes.npy"), n.astype(np.float64))
+    np.save(os.path.join(out_dir, "sketch_hashes_hi.npy"), (h >> np.uint64(32)).astype(np.float64))
+    np.save(os.path.join(out_dir, "sketch_hashes_lo.npy"), (h & np.uint64(0xFFFFFFFF)).astype(np.float64))
 
 
 def measured_peaks():
@@ -635,6 +658,8 @@ def main():
                                  "alu_pipe_frac": warp_inst * model["alu_pipe_share"] / (issue_peak / 2),
                                  "note": "ALU pipe (SHF/LOP3/IADD3/PRMT) issues one warp instruction per 2 clocks per sub-partition; instruction mix from the ncu source page"}
     sanity = {"sketches_full": int((d_n == S).sum().item()), "units": n_units}
+    if args.dump_outputs and rank == 0:
+        dump_sketch_outputs(args.dump_outputs, d_hashes, d_n)
 
     # ---------------- e2e: host buffers through mashgpu_sketch_batch --------------------------------------------------
     e2e = None
@@ -783,12 +808,11 @@ def main():
         eng.set_timing(True); eng.stats(reset=True)
         barrier()
         e0.record(st)
-        dK = min(Ksteps, 2) if n_ref * n_qry >= 10 ** 9 else Ksteps
-        for _ in range(dK):
+        for _ in range(Ksteps):
             dist_step()
         e1.record(st)
         barrier()
-        dms = max_over_ranks(e0.elapsed_time(e1)) / dK
+        dms = max_over_ranks(e0.elapsed_time(e1)) / Ksteps
         dstats = eng.stats(reset=True)
         eng.set_timing(False)
         pairs_per_rank = n_ref * n_qry
@@ -826,7 +850,7 @@ def main():
                    "ms": a0.elapsed_time(a1), "pairs_per_s": tri_pairs / (a0.elapsed_time(a1) * 1e-3)}
             job.set_triangle(False)
         dist_obj = {"metric": "sketch_pairs_per_s", "value": total_pairs / (dms * 1e-3), "unit": "pairs/s", "ms_per_step": dms,
-                    "steps": dK, "warmup": dW, "pairs_per_step": total_pairs, "enumeration": "all ordered pairs (full Q x R grid)",
+                    "steps": Ksteps, "warmup": dW, "pairs_per_step": total_pairs, "enumeration": "all ordered pairs (full Q x R grid)",
                     "workload": f"configs[2]: {n_sk} synthetic s={S} sketches all-vs-all, 100 families stored family by family (SURVEY.md 8d generator); "
                                 f"reference axis sharded over {world} rank(s), every rank compares all {n_sk} queries with its shard",
                     "outputs": "dense numer,denom (u32), distance,pvalue (f64), pass (u8) = 25 B/pair written to an HBM tile buffer that is reused per query tile",
@@ -841,9 +865,9 @@ def main():
                                 "sharded dictionary build: local sort, all-to-all by hash range, ranking, all-to-all back, all-gather of the encoded rows "
                                 "(mash_b200/shard.py sharded_dictionary), then mashgpu_dist_open_encoded; wall clock, max over ranks"),
                     "sharded_dictionary": dstat,
-                    "kernel_ms_per_step": dstats["dist_kernel_ms"] / dK, "gpu_launches": int(dstats["kernel_launches"]),
+                    "kernel_ms_per_step": dstats["dist_kernel_ms"] / Ksteps, "gpu_launches": int(dstats["kernel_launches"]),
                     "pairs_with_shared_hashes_in_last_tile": last_shared_nonzero,
-                    "roofline": {"bound": "hbm", "achieved": (total_pairs / world * 25 + (n_ref + n_qry) * S * 4) / (dstats["dist_kernel_ms"] / dK * 1e-3) / 1e9,
+                    "roofline": {"bound": "hbm", "achieved": (total_pairs / world * 25 + (n_ref + n_qry) * S * 4) / (dstats["dist_kernel_ms"] / Ksteps * 1e-3) / 1e9,
                                  "peak": peaks["hbm_gbs"], "unit": "GB/s",
                                  "note": "algorithmic bytes = 25 B/pair written + the rank rows read once; the probe kernel is ALU-pipe bound and the merge "
                                          "kernel shared-memory bound, not HBM bound (DESIGN.md 3.3)"}}

@@ -95,6 +95,36 @@ class Golden:
         return np.array(s["hashes"], dtype=np.uint64), s["length"]
 
 
+class ReferenceAnswers:
+    """What the reference's own code answered for the inputs of a test module, stored in tests/golden/<name>.npz so that the
+    comparison runs in every checkout.  `answers(key, compute)` returns the stored answer; when recording (reference given,
+    `pytest --record-reference`), it returns compute(reference) instead and save() writes the file.  Changing a test's inputs
+    means recording again where the reference can be built (oracle/Makefile)."""
+
+    def __init__(self, name, reference=None):
+        self.path = os.path.join(GOLDEN, name + ".npz")
+        self.reference = reference
+        self.stored = dict(np.load(self.path)) if os.path.exists(self.path) else {}
+
+    def __call__(self, key, compute):
+        if self.reference is not None:
+            out = compute(self.reference)
+            for i, v in enumerate(out if isinstance(out, tuple) else (out,)):
+                self.stored[f"{key}.{i}"] = np.asarray(v)
+            return out
+        if f"{key}.0" not in self.stored:
+            raise KeyError(f"{self.path} holds no answer for {key!r}: record it with `pytest --record-reference`")
+        out = []
+        while f"{key}.{len(out)}" in self.stored:
+            v = self.stored[f"{key}.{len(out)}"]
+            out.append(v.item() if v.ndim == 0 else v)
+        return tuple(out) if len(out) > 1 else out[0]
+
+    def save(self):
+        if self.reference is not None:
+            np.savez_compressed(self.path, **self.stored)
+
+
 def fmt_g(x):
     """iostream default formatting of a double: %g with 6 significant digits."""
     return "%g" % x

@@ -8,11 +8,15 @@
     (oracle/_ref/libmash_ref.so -> getHash, hash.cpp:10-38)
   * pvalue_mpmath.json: 50-digit mpmath values of P[Bin(n, r) >= x] = I_r(x, n-x+1), the quantity
     gsl_cdf_binomial_Q(x-1, r, n) evaluates (CommandDistance.cpp:446, CommandScreen.cpp:613)
+  * ref_objcode.npz, ref_kseq.npz: the answers of the reference's object code (oracle/_ref/libmash_ref.so) and of its parser
+    (oracle/_ref/kseq_dump) for the inputs of tests/test_oracle_vs_ref.py and tests/test_host_fastx_vs_kseq.py, recorded by
+    running those tests with --record-reference
 """
 import gzip
 import json
 import os
 import shutil
+import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -71,6 +75,9 @@ def main():
         v = mp.betainc(x, n - x + 1, 0, mp.mpf(r), regularized=True)
         cases.append(dict(x=x, r=repr(float(r)), n=n, p=mp.nstr(v, 25)))
     json.dump(cases, open(os.path.join(HERE, "pvalue_mpmath.json"), "w"), indent=0)
+
+    subprocess.check_call([sys.executable, "-m", "pytest", "-q", "--record-reference",
+                           "tests/test_oracle_vs_ref.py", "tests/test_host_fastx_vs_kseq.py"], cwd=ROOT)
     print("golden fixtures written:", sorted(os.listdir(HERE)))
 
 
