@@ -11,7 +11,6 @@ struct SketchStream {
     const uint32_t *d_inval = nullptr;      // ... and the invalid-position bit mask (see pack.cpp)
     const uint64_t *unit_start = nullptr;   // host, n_units + 1
     uint64_t n_units = 0;
-    bool force_keep_all = false;
     cudaEvent_t data_ready = nullptr;       // when set: the scan kernel waits for this event (an upload on another stream); the parameter
                                             // copies of the pass are enqueued before the wait -- they come from pageable memory and would
                                             // otherwise hold the calling thread until the upload has finished
@@ -40,8 +39,8 @@ struct SketchTicket {
     std::vector<uint64_t> unit_start;       // own copy of S.unit_start
     uint64_t *d_out_hashes = nullptr; uint32_t *d_out_counts = nullptr, *d_out_n = nullptr;
     cudaStream_t st = nullptr;
+    uint32_t min_copies = 1;                // `-m` of the tables (1 for the screen mixture), the same in the re-runs
     uint64_t *d_qtarget = nullptr, *d_qtstar = nullptr;
-    std::vector<uint8_t> scan_args;         // the ScanArgs of the pass (base of the re-runs), kept opaque here
 };
 
 int validate_sketch_params(mashgpu_ctx *ctx, const mashgpu_sketch_params *p);

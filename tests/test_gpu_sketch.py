@@ -278,8 +278,8 @@ def test_feed_scheduler_many_waves_pinned_buffers(gpu, oracle, monkeypatch, mode
 
 
 def test_large_sketch_size_goes_through_global_sort(gpu, oracle):
-    # s = 5000: the unit's candidate table (2^16 slots) does not fit select_kernel's shared-memory sort, so the unit takes
-    # the exact re-run path (global-memory table + radix sort) -- same answer, `mash sketch -s 5000`
+    # s = 5000: the unit's candidate table (2^16 slots) does not fit select_kernel's shared-memory sort, so the unit goes
+    # through the segmented radix sort -- same answer, `mash sketch -s 5000`
     p = gpu.params(k=21, s=5000)
     po = oracle.params(k=21)
     g = bytes(synth_genome(1234, 400_000))
